@@ -4,6 +4,7 @@ ms to logpdf(fx,y) + posterior(fx,y) at N x D fp64, with the achieved fraction o
 trailing update and of the N^3/3 Cholesky rate, next to the reference's CPU LAPACK path timed on the same box.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C2|C4h|C3|C5] [--impl ours|reference] [--n N]
+                  [--dump-outputs DIR]
 
 The SAME workload (C4: N = 65 536, D = 64, SqExponential, fp64 -- the configuration BASELINE.json's metric and target are
 quoted on; it fits one B200) runs at every --gpus value, so the per-N values form a strong-scaling curve.  At N = 1 the
@@ -16,6 +17,10 @@ One "step" = one pass of the hot path through the C ABI of libagp.so:
 HOST buffers, H2D/D2H inside the timed region.  Device times come from CUDA events recorded by the library on its
 launching stream, max over ranks.  The oracle (oracle/agp_ref.py) is used here only as the CPU baseline and as the
 out-of-timed-region parity checker.
+
+--dump-outputs DIR writes what the last device-resident timed step returned to its caller as DIR/<name>.npy (logpdf and
+alpha; mean and var for C3; elbo and dtc for C5), so two builds can be compared output for output on the same seeded
+inputs.  An array too large for the 64 MB budget is replaced by a fixed seeded sample of its entries.
 """
 from __future__ import annotations
 
@@ -31,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # a benchmark run leaves the tree as it found it (it may be read-only)
 
 WORKLOADS = {  # BASELINE.json configs (SURVEY.md s8d)
     "C2": dict(kind="fit", N=4096, D=8, dtype="f64", kernel="SqExponential", s2=0.1, cfg="C2"),
@@ -42,6 +48,7 @@ WORKLOADS = {  # BASELINE.json configs (SURVEY.md s8d)
 METRIC = {"fit": "ms to logpdf(fx,y)+posterior(fx,y)", "fit_predict": "ms to logpdf+posterior+mean_and_var(10000 test points)",
           "vfe": "ms to elbo(VFE(f(z)), fx, y)"}
 CPU_SUB = 8192  # bounded CPU sample for the cubic workloads (scaled by (N/8192)^3, labelled extrapolated)
+DUMP_BYTES = 64 * 10 ** 6  # everything --dump-outputs writes, .npy headers included
 
 
 def make_inputs(wl, n=None):
@@ -382,6 +389,28 @@ class FitProblem:
             L.agp_post_free(post)
         return t
 
+    def outputs(self):
+        """host copies of what the last device-resident step returned (scalars land in host memory in either mode)"""
+        self.torch.cuda.synchronize()
+        if self.kind == "vfe":
+            return {"elbo": self.lp[0:1].copy(), "dtc": self.lp[1:2].copy()}
+        out = {"logpdf": self.lp[0:1].copy(), "alpha": self.alpha_d.cpu().numpy()}
+        if self.kind == "fit_predict":
+            out["mean"], out["var"] = self.mu_d.cpu().numpy(), self.var_d.cpu().numpy()
+        return out
+
+
+def dump_outputs(outs, d):
+    """DIR/<name>.npy per output, within DUMP_BYTES in all; a larger array keeps a fixed seeded sample of its entries"""
+    os.makedirs(d, exist_ok=True)
+    per = (DUMP_BYTES - 1024 * len(outs)) // len(outs)
+    for name, a in outs.items():
+        a = np.ascontiguousarray(a).reshape(-1)
+        cap = per // a.itemsize
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+
 
 def timed(prob, torch, flush, device_resident, steps, warmup, dist=None):
     eng = prob.eng
@@ -460,7 +489,8 @@ def fit_roofline(wl, N, eng, torch, dev, prob, flush, args, world=1, dist=None, 
         eng.set_config(lookahead=0, profile_kernels=1)
     else:
         eng.set_config(profile_kernels=1)
-    t_serial, _, _ = timed(prob, torch, flush, True, max(2, min(args.steps, 3)), 1, dist)
+    roof_steps = min(args.steps, 3)
+    t_serial, _, _ = timed(prob, torch, flush, True, roof_steps, 1, dist)
     eng.set_config(lookahead=cfg0.lookahead, profile_kernels=cfg0.profile_kernels)
     n_pad = (N + 127) // 128 * 128
     nb = cfg0.tile_nb if cfg0.tile_nb > 0 else (512 if n_pad >= 8192 else 128)
@@ -473,7 +503,7 @@ def fit_roofline(wl, N, eng, torch, dev, prob, flush, args, world=1, dist=None, 
     trailing_ms = t_serial.get("trailing", 0.0)  # max over ranks of the per-rank sum of launch durations
     out = {"launches_per_step": launches * world, "alg_flops_per_step": tf, "kernel_ms_per_step": trailing_ms,
            "kernel_ms_per_step_rank_max": trailing_ms, "panel_width": nb,
-           "kernel_timing": "CUDA events around each launch%s, %d steps" % (", look-ahead off (serial)" if dist is None else ", max over ranks of the per-rank sum", max(2, min(args.steps, 3)))}
+           "kernel_timing": "CUDA events around each launch%s, %d steps" % (", look-ahead off (serial)" if dist is None else ", max over ranks of the per-rank sum", roof_steps)}
     if W["dtype"] == "f64" and mode == 1:
         pairs = S_sl * (S_sl + 1) // 2
         fp64_eq = tf / world / (trailing_ms * 1e-3) / 1e12 if trailing_ms > 0 else None  # per GPU
@@ -556,6 +586,8 @@ def run_ours(args, wl, n_full):
     if rank == 0:
         sampler.start()
     t_dev, wall_dev, launches = timed(prob, torch, flush, True, args.steps, args.warmup, dist)
+    if args.dump_outputs and rank == 0:  # before the passes below reuse the problem's buffers
+        dump_outputs(prob.outputs(), args.dump_outputs)
     if args.quick:  # development runs (schedule sweeps): device-resident timing only, no e2e / parity / roofline / CPU arm
         if rank == 0:
             sampler.stop()
@@ -631,7 +663,7 @@ def run_ours(args, wl, n_full):
 def secondary_c2(eng, torch, dev, flush, args):
     """BASELINE config C2 (N = 4096, D = 8): latency-bound single-GPU case, carried next to the C4 headline"""
     p = FitProblem("C2", None, eng, torch, dev)
-    steps = max(5, min(args.steps, 20))
+    steps = min(args.steps, 20)
     t_dev, _, launches = timed(p, torch, flush, True, steps, 3)
     t_e2e, _, _ = timed(p, torch, flush, False, steps, 3)
     par = None
@@ -654,7 +686,13 @@ def main():
     ap.add_argument("--n", type=int, default=None, help="override N of the workload (development / shard-sized runs)")
     ap.add_argument("--no-c2", action="store_true", help="skip the secondary C2 measurement on the N=1 C4 line")
     ap.add_argument("--quick", action="store_true", help="development: device-resident timing only (not a bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last device-resident timed step returned as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "ours":
         args.warmup = max(args.warmup, 3)
     wl = args.workload

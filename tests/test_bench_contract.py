@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -53,3 +56,36 @@ def test_roofline_traffic_record_is_committed():
         assert t and t["dram_bytes_per_launch"] > 0 and t["algorithmic_bytes_per_launch"] > 0
         assert 1.0 <= t["ratio"] < 1.5, t["ratio"]          # traffic close to the algorithmic bytes: no wasted re-reads
         assert os.path.exists(os.path.join(ROOT, t["capture"]))
+
+
+def test_dump_outputs_fits_budget_with_a_fixed_sample(tmp_path):
+    """--dump-outputs: one float .npy per output, all of them within DUMP_BYTES; an oversized output is replaced by the
+    same seeded sample of its entries on every run"""
+    sys.path.insert(0, ROOT)
+    import bench
+    outs = {"logpdf": np.array([-1.5]), "alpha": np.arange(bench.DUMP_BYTES // 8 + 10, dtype=np.float64)}
+    for d in ("a", "b"):
+        bench.dump_outputs(outs, str(tmp_path / d))
+    sizes = [os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")]
+    assert sorted(os.listdir(tmp_path / "a")) == ["alpha.npy", "logpdf.npy"] and sum(sizes) <= bench.DUMP_BYTES
+    a, b = np.load(tmp_path / "a" / "alpha.npy"), np.load(tmp_path / "b" / "alpha.npy")
+    assert a.dtype == np.float64 and 0 < a.size < outs["alpha"].size and np.array_equal(a, b)
+    assert np.all(np.diff(a) > 0)  # sampled entries keep their order
+    assert np.load(tmp_path / "a" / "logpdf.npy").tolist() == [-1.5]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_match_oracle(tmp_path, ref):
+    """bench.py --dump-outputs on C2 writes the logpdf and alpha of its last timed step; they match the oracle"""
+    out = tmp_path / "out"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "C2", "--steps", "2", "--warmup", "1",
+                        "--quick", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    cfg = ref.make_config("C2")
+    lp = np.load(out / "logpdf.npy")
+    alpha = np.load(out / "alpha.npy")
+    lp_ref = ref.logpdf(cfg["k"], cfg["mean"], cfg["noise"], cfg["X"], cfg["y"])
+    alpha_ref = ref.posterior(cfg["k"], cfg["mean"], cfg["noise"], cfg["X"], cfg["y"])["alpha"]
+    assert lp.dtype == np.float64 and lp.shape == (1,) and abs(lp[0] - lp_ref) <= 1e-8 * abs(lp_ref)
+    assert alpha.shape == (4096,) and np.allclose(alpha, alpha_ref, rtol=1e-7, atol=1e-9)
